@@ -2,6 +2,7 @@
 """bench.py -- POA windows/sec of the B200-native engine (BASELINE.json metric).
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (+ the last timed step's results, see dump_outputs)
     python bench.py --impl reference --gpus N --steps K --warmup W
 
 Headline workload (config.workload): BASELINE.json configs[1] -- "single B200: 10k windows, 500 bp x 32 reads,
@@ -205,8 +206,9 @@ def run_reference(args, rank, world):
     }))
 
 
-def measure(name, args, rank, world, local_rank, device, steps, warmup, nwin=None, sample_clocks=True):
-    """Kernel-only and end-to-end legs of one workload on this rank.  Returns a dict of per-rank raw numbers."""
+def measure(name, args, rank, world, local_rank, device, steps, warmup, nwin=None, sample_clocks=True, keep_outputs=False):
+    """Kernel-only and end-to-end legs of one workload on this rank.  Returns a dict of per-rank raw numbers (and, with
+    keep_outputs, what each leg's last timed step returned)."""
     import torch
     import torch.distributed as dist
     from racon_gpu_b200 import api
@@ -254,7 +256,7 @@ def measure(name, args, rank, world, local_rank, device, steps, warmup, nwin=Non
         clocks = sampler.stop() if sample_clocks else None
     dev_ms = float(sum(a.elapsed_time(b) for a, b in ev))
     pb.download()
-    _, _, status_k = pb.get_consensus()
+    cons_k, cov_k, status_k = pb.get_consensus()
     n_fail = int((status_k != 0).sum())
     pb.close()
 
@@ -292,9 +294,44 @@ def measure(name, args, rank, world, local_rank, device, steps, warmup, nwin=Non
     n_unpolished = int((~polished).sum())
     pol.close()
     arena.close()
-    return {"batch": batch, "nwin": nwin, "L": L, "banded": banded, "info": info, "dev_ms": dev_ms, "e2e_s": e2e_s,
-            "wall": wall, "failures": n_fail + n_unpolished, "h2d": h2d, "d2h": d2h, "clocks": clocks,
-            "launches": steps + warmup + e2e_launches, "timed_launches": steps + e2e_launches}
+    out = {"batch": batch, "nwin": nwin, "L": L, "banded": banded, "info": info, "dev_ms": dev_ms, "e2e_s": e2e_s,
+           "wall": wall, "failures": n_fail + n_unpolished, "h2d": h2d, "d2h": d2h, "clocks": clocks,
+           "launches": steps + warmup + e2e_launches, "timed_launches": steps + e2e_launches}
+    if keep_outputs:
+        out["outputs"] = {"kernel": (cons_k, cov_k, status_k), "e2e": (cons, clen, polished, status)}
+    return out
+
+
+DUMP_BYTES = 63_000_000  # data of all --dump-outputs files; the .npy headers stay within 64 MB with it
+
+
+def dump_outputs(out_dir, outputs):
+    """--dump-outputs: the results of the last timed step as float32 .npy files.  Kernel leg (the headline `value`):
+    what PoaBatch.get_consensus returns -- untrimmed consensus, its per-base coverage, status per window.  e2e leg: what
+    Polisher.polish_arena returns -- trimmed consensus, polished flag, status per window.  Consensus and coverage are
+    concatenated over windows, with the lengths beside them.  When the worst case of all windows (every consensus as
+    long as the output stride) would exceed DUMP_BYTES, a fixed seeded sample of windows is written (window_index)."""
+    cons_k, cov_k, status_k = outputs["kernel"]
+    cons_e, clen_e, polished_e, status_e = outputs["e2e"]
+    nwin, stride = len(cons_k), cons_e.shape[1]
+    per_window = 4 * (3 * stride + 6)
+    idx = np.arange(nwin)
+    if nwin * per_window > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(nwin, DUMP_BYTES // per_window, replace=False))
+    arrays = {
+        "window_index": idx,
+        "consensus": np.frombuffer(b"".join(cons_k[i] for i in idx), dtype=np.uint8),
+        "consensus_length": np.asarray([len(cons_k[i]) for i in idx]),
+        "coverage": np.concatenate([cov_k[i] for i in idx]),
+        "status": status_k[idx],
+        "e2e_consensus": np.concatenate([cons_e[i, :clen_e[i]] for i in idx]),
+        "e2e_consensus_length": clen_e[idx],
+        "e2e_polished": polished_e[idx],
+        "e2e_status": status_e[idx],
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 def measure_msa(args, local_rank, device, steps=3, warmup=3):
@@ -487,7 +524,11 @@ def main():
     ap.add_argument("--rounds", type=float, default=1.0, help="e2e leg: launches per batch processor per step (chunk = windows / (batches x rounds))")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the A_full / B_banded block (N=1 only anyway)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's windows) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -508,7 +549,8 @@ def main():
         dist.init_process_group("nccl", device_id=device)
     warmup = max(args.warmup, 3)
 
-    m = measure(args.workload, args, rank, world, local_rank, device, args.steps, warmup, nwin=args.windows or None)
+    m = measure(args.workload, args, rank, world, local_rank, device, args.steps, warmup, nwin=args.windows or None,
+                keep_outputs=bool(args.dump_outputs) and rank == 0)
 
     # ---------------- reduce over ranks ---------------------------------------------------------------
     dev_ms, e2e_s, wall, failures = m["dev_ms"], m["e2e_s"], m["wall"], m["failures"]
@@ -525,6 +567,8 @@ def main():
             dist.destroy_process_group()
         return
 
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, m.pop("outputs"))
     nwin, info = m["nwin"], m["info"]
     total_windows = nwin * world
     m["dev_ms"] = dev_ms

@@ -21,5 +21,5 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def ref():
-    from oracle_lib import Ref
-    return Ref()
+    from oracle_lib import RefAnswers
+    return RefAnswers()

@@ -1,12 +1,14 @@
 """ctypes loaders for the parity checkers (TEST INFRASTRUCTURE: tests/, smoke(), bench cpu legs only).
 
-  Oracle  -> oracle/liboracle.so          plain-C restatement of racon's spoa path
-  Ref     -> oracle/_ref/libracon_ref.so  the unmodified reference (racon::Window + spoa), built
-                                          here from /root/reference by oracle/Makefile
+  Oracle      -> oracle/liboracle.so          plain-C restatement of racon's spoa path
+  Ref         -> oracle/_ref/libracon_ref.so  the unmodified reference (racon::Window + spoa + edlib), built
+                                              from racon's sources by oracle/Makefile
+  RefAnswers  -> tests/golden/ref_answers.npz what Ref answered for the inputs the tests ask it about
 """
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -14,6 +16,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
+REF_ANSWERS = os.path.join(ROOT, "tests", "golden", "ref_answers.npz")
 
 
 def build_oracle(quiet: bool = True) -> None:
@@ -244,3 +247,120 @@ def ref_breaking_points(ref: "Ref", cigar: bytes, q_length: int, q_begin: int, q
                                           C.c_uint32(window_length), _p(out, C.c_uint32), C.c_int64(cap))
     assert n >= 0
     return out[:2 * n].reshape(-1, 2).copy()
+
+
+# ---------------------------------------------------------------------------------------------------
+# stored answers of the unmodified reference: the comparisons with it run where oracle/_ref cannot be built
+# ---------------------------------------------------------------------------------------------------
+def _digest(kind: str, *parts) -> str:
+    h = hashlib.sha256()
+    for p in parts:
+        if isinstance(p, np.ndarray):
+            h.update(b"a%s%s:" % (p.dtype.str.encode(), str(p.shape).encode()))
+            h.update(np.ascontiguousarray(p).tobytes())
+        elif isinstance(p, (bytes, bytearray)):
+            h.update(b"b%d:" % len(p))
+            h.update(bytes(p))
+        elif isinstance(p, (list, tuple)):
+            h.update(b"l%d:" % len(p))
+            h.update(_digest("", *p).encode())
+        elif p is None:
+            h.update(b"n")
+        else:
+            h.update(b"i%d" % int(p))
+        h.update(b"|")
+    return kind + "_" + h.hexdigest()[:32]
+
+
+class RefAnswers:
+    """The answers of the unmodified reference (Ref) to the questions the tests ask it, with Ref's call signatures.
+
+    Replay (default): answers come from tests/golden/ref_answers.npz, keyed by a digest of the question's inputs; a
+    question it has no answer for raises KeyError.  Recording (RefAnswers(Ref())): every question goes to the live
+    reference and its answer is kept for save() -- tests/golden/make_ref_answers.py."""
+
+    def __init__(self, live: Ref | None = None):
+        self.live = live
+        self.store = {} if live is not None else self._load(REF_ANSWERS)
+
+    def _answer(self, key, fields, ask):
+        if self.live is not None:
+            for f, v in zip(fields, ask()):
+                self.store[(key, f)] = np.asarray(v)
+        try:
+            return [self.store[(key, f)] for f in fields]
+        except KeyError:
+            raise KeyError(f"{key}: no stored answer of the reference for these inputs "
+                           f"(tests/golden/make_ref_answers.py records them)") from None
+
+    # on disk: per (question kind, field) one array of all answers concatenated, their keys and their shapes
+    def save(self, path: str = REF_ANSWERS):
+        groups = {}
+        for (key, f), a in sorted(self.store.items()):
+            groups.setdefault(key.split("_")[0] + "_" + f, []).append((key, a))
+        out = {}
+        for g, items in groups.items():
+            out[g + "_keys"] = np.asarray([k for k, _ in items], dtype="S")
+            out[g + "_shapes"] = np.asarray([(a.ndim,) + a.shape + (1,) * (2 - a.ndim) for _, a in items], dtype=np.int64)
+            out[g] = np.concatenate([a.reshape(-1) for _, a in items])
+        np.savez_compressed(path, **out)
+
+    @staticmethod
+    def _load(path):
+        z = np.load(path)
+        store = {}
+        for g in (n[:-5] for n in z.files if n.endswith("_keys")):
+            f = g.split("_", 1)[1]
+            data, at = z[g], 0
+            for k, (ndim, rows, cols) in zip(z[g + "_keys"], z[g + "_shapes"]):
+                store[(k.decode(), f)] = data[at:at + rows * cols].reshape((rows, cols)[:ndim])
+                at += rows * cols
+        return store
+
+    def layer_order(self, begins: np.ndarray) -> np.ndarray:
+        begins = np.ascontiguousarray(begins, dtype=np.int32)
+        return self._answer(_digest("order", begins), ["rank"], lambda: [self.live.layer_order(begins)])[0]
+
+    def polish(self, batch, m: int, x: int, g: int, tgs: bool = True, trim: bool = True,
+               threads: int = 1, window_length: int = 500):
+        key = _digest("polish", batch.win_seq_off, batch.seq_off, batch.bases, batch.weights, batch.has_weights,
+                      batch.begins, batch.ends, m, x, g, tgs, trim, window_length)
+
+        def ask():
+            cons, pol = self.live.polish(batch, m, x, g, tgs=tgs, trim=trim, threads=threads, window_length=window_length)
+            return [np.frombuffer(b"\n".join(cons), dtype=np.uint8), pol.astype(np.uint8)]
+        cons, pol = self._answer(key, ["cons", "polished"], ask)
+        return cons.tobytes().split(b"\n"), pol.astype(bool)
+
+    def spoa_window(self, seqs, weights, m: int, x: int, g: int):
+        key = _digest("spoa", [bytes(s) for s in seqs], list(weights), m, x, g)
+
+        def ask():
+            cons, cov, rank = self.live.spoa_window(seqs, weights, m, x, g)
+            return [np.frombuffer(cons, dtype=np.uint8), cov, rank]
+        cons, cov, rank = self._answer(key, ["cons", "cov", "rank"], ask)
+        return cons.tobytes(), cov, rank
+
+    def window_msa(self, seqs, weights, m: int, x: int, g: int):
+        """ref_window_msa: the MSA rows of one group."""
+        key = _digest("msa", [bytes(s) for s in seqs], list(weights), m, x, g)
+
+        def ask():
+            rows = ref_window_msa(self.live, seqs, weights, m, x, g)
+            return [np.frombuffer(b"".join(rows), dtype=np.uint8).reshape(len(rows), -1)]
+        return [r.tobytes() for r in self._answer(key, ["rows"], ask)[0]]
+
+    def align(self, q: bytes, t: bytes):
+        """ref_align: (ops, edit distance, CIGAR) of edlib called like racon calls it."""
+        def ask():
+            ops, score, cigar = ref_align(self.live, q, t)
+            return [ops, score, np.frombuffer(cigar, dtype=np.uint8)]
+        ops, score, cigar = self._answer(_digest("aln", q, t), ["ops", "score", "cigar"], ask)
+        return ops, int(score), cigar.tobytes()
+
+    def breaking_points(self, cigar: bytes, q_length: int, q_begin: int, q_end: int, strand: int, t_length: int,
+                        t_begin: int, t_end: int, window_length: int):
+        """ref_breaking_points: (t, q) pairs of racon::Overlap::find_breaking_points fed this CIGAR."""
+        args = (q_length, q_begin, q_end, strand, t_length, t_begin, t_end, window_length)
+        return self._answer(_digest("bp", cigar, *args), ["points"],
+                            lambda: [ref_breaking_points(self.live, cigar, *args)])[0]

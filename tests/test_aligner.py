@@ -2,15 +2,16 @@
 
 Parity target = the CIGAR racon's CPU path gets from edlib (NW, path).  Here: the oracle's restatement
 (oracle/aln_oracle.c) against the committed digests of the unmodified edlib on REAL overlaps
-(tests/golden/lambda_overlaps.npz), live against oracle/_ref on random pairs around every threshold of edlib's
-recursion, and the engine's lane emulation against the oracle.  GPU: tests/test_gpu_aligner.py."""
+(tests/golden/lambda_overlaps.npz), against its stored answers (tests/golden/ref_answers.npz) on random pairs around
+every threshold of edlib's recursion, and the engine's lane emulation against the oracle.  GPU:
+tests/test_gpu_aligner.py."""
 import hashlib
 
 import numpy as np
 import pytest
 
 from common import overlap_fixture, random_pairs
-from oracle_lib import ops_to_cigar, oracle_align, ref_align
+from oracle_lib import ops_to_cigar, oracle_align
 
 SHAPES = [(1, 0.5), (2, 0.5), (5, 0.3), (63, 0.2), (64, 0.2), (65, 0.2), (129, 0.25), (200, 0.15), (700, 0.15),
           (1500, 0.1), (1800, 0.15), (1850, 0.15), (2000, 0.15), (2600, 0.2), (4000, 0.12), (5000, 0.3)]
@@ -28,8 +29,6 @@ def test_restatement_matches_edlib_digests_on_real_overlaps(oracle):
 
 
 def test_restatement_matches_live_edlib(oracle, ref):
-    if not ref.available:
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
     pairs = []
     for rep in range(6):
         pairs += random_pairs(100 + rep, [s for s in SHAPES if s[0] < 300 or rep < 2])
@@ -39,7 +38,7 @@ def test_restatement_matches_live_edlib(oracle, ref):
                       rng.choice(np.frombuffer(b"ACGT", dtype=np.uint8), size=m).tobytes()))
     for q, t in pairs:
         a, sa = oracle_align(oracle, q, t)
-        b, sb, cigar = ref_align(ref, q, t)
+        b, sb, cigar = ref.align(q, t)
         assert sa == sb and a.shape == b.shape and (a == b).all()
         assert ops_to_cigar(oracle, a) == cigar
 
@@ -91,25 +90,23 @@ def test_emulated_aligner_on_real_overlaps(oracle, emu):
 def test_emulated_aligner_on_long_reads_against_live_edlib(ref, emu):
     """40 kb reads: five Hirschberg levels, all three shape classes (short / tall / huge), leaves of many stripes; only
     the real edlib is fast enough to be the checker here."""
-    if not ref.available:
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
     pairs = random_pairs(902, [(42000, 0.12)])
     rng = np.random.default_rng(5)
     acgt = np.frombuffer(b"ACGT", dtype=np.uint8)
     pairs.append((rng.choice(acgt, size=30000).tobytes(), rng.choice(acgt, size=12000).tobytes()))
     pairs.append((rng.choice(acgt, size=900).tobytes(), rng.choice(acgt, size=50000).tobytes()))
     for q, t in pairs:
-        ops, score, cigar = ref_align(ref, q, t)
+        ops, score, cigar = ref.align(q, t)
         a, sa, depth, leaves = emu.align(q, t)
         assert sa == score and a.shape == ops.shape and (a == ops).all() and emu.cigar == cigar
     assert depth >= 3
 
 
 def test_breaking_points_restatement_and_engine(oracle, ref, emu):
-    """src/overlap.cpp:226-290: the oracle's restatement against the UNMODIFIED racon (oracle/_ref) on random overlaps
-    with random coordinates / strands / window lengths, the committed real breaking points (window length 500), and the
-    engine's run-based version (lane emulation) against both."""
-    from oracle_lib import oracle_breaking_points, ref_breaking_points
+    """src/overlap.cpp:226-290: the oracle's restatement against the UNMODIFIED racon (its stored answers) on random
+    overlaps with random coordinates / strands / window lengths, the committed real breaking points (window length 500),
+    and the engine's run-based version (lane emulation) against both."""
+    from oracle_lib import oracle_breaking_points
     rng = np.random.default_rng(3)
     for rep in range(60):
         n, e = int(rng.integers(1, 3000)), float(rng.uniform(0.02, 0.4))
@@ -121,10 +118,9 @@ def test_breaking_points_restatement_and_engine(oracle, ref, emu):
         q_first = q_len - (q_begin + len(q)) if strand else q_begin
         ops, score = oracle_align(oracle, q, t)
         want = oracle_breaking_points(oracle, ops, q_first, t_begin, t_begin + len(t), w)
-        if ref.available:
-            got = ref_breaking_points(ref, ops_to_cigar(oracle, ops), q_len, q_begin, q_begin + len(q), strand,
-                                      t_begin + len(t) + 5, t_begin, t_begin + len(t), w)
-            assert got.shape == want.shape and (got == want).all(), rep
+        got = ref.breaking_points(ops_to_cigar(oracle, ops), q_len, q_begin, q_begin + len(q), strand,
+                                  t_begin + len(t) + 5, t_begin, t_begin + len(t), w)
+        assert got.shape == want.shape and (got == want).all(), rep
         emu.align(q, t, q_first, t_begin, w)
         assert emu.breaking_points.shape == want.shape and (emu.breaking_points == want).all(), (rep, n, w)
     fx = overlap_fixture()
@@ -152,9 +148,9 @@ def test_banded_passes_with_guessed_and_exact_bounds(oracle, ref, emu):
         for guess in (0, score // 2, score - 1, score, score + 1, 2 * score + 64, 10 ** 6):
             a, sa, depth, leaves = emu.align(q, t, guess=guess)
             assert sa == score and a.shape == ops.shape and (a == ops).all(), (len(q), len(t), guess)
-    if ref.available:  # long reads: narrow strips of a large matrix, several stripes handing over anchors
-        for (q, t), frac in zip(random_pairs(903, [(42000, 0.12), (30000, 0.03)]), (0.25, 0.05)):
-            ops, score, cigar = ref_align(ref, q, t)
-            for guess in (int(frac * len(t)), score, score - 1):
-                a, sa, depth, leaves = emu.align(q, t, guess=guess)
-                assert sa == score and (a == ops).all() and emu.cigar == cigar, (len(q), guess)
+    # long reads: narrow strips of a large matrix, several stripes handing over anchors
+    for (q, t), frac in zip(random_pairs(903, [(42000, 0.12), (30000, 0.03)]), (0.25, 0.05)):
+        ops, score, cigar = ref.align(q, t)
+        for guess in (int(frac * len(t)), score, score - 1):
+            a, sa, depth, leaves = emu.align(q, t, guess=guess)
+            assert sa == score and (a == ops).all() and emu.cigar == cigar, (len(q), guess)

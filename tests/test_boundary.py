@@ -1,9 +1,10 @@
 """CPU: the drop-in boundary claim of INTEGRATION.md section 2, checked against the reference's own adapter source.
 
-A temporary copy of /root/reference/src/cuda/cudabatch.{hpp,cpp} receives ONLY the textual changes INTEGRATION.md
+A temporary copy of racon's src/cuda/cudabatch.{hpp,cpp} receives ONLY the textual changes INTEGRATION.md
 shows (include of the shim, the cudapoa namespace) and must then compile (`g++ -fsyntax-only -DCUDA_ENABLED`)
 against racon_gpu_b200/csrc/host/b200poa_batch.hpp -- racon's adapter is the FFI of this path, so this is the
-"binding builds" check.  Skipped where /root/reference does not exist (the GPU box)."""
+"binding builds" check.  racon's sources are taken where oracle/Makefile builds the reference from (its REF, which
+the environment can override); skipped where they are not present."""
 import os
 import shutil
 import subprocess
@@ -11,10 +12,12 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = subprocess.run(["make", "-s", "--no-print-directory", "-C", os.path.join(ROOT, "oracle"), "print-ref"],
+                     capture_output=True, text=True).stdout.strip()
+NO_SOURCES = not (REF and os.path.isdir(os.path.join(REF, "src", "cuda")))
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src", "cuda")), reason="reference sources not present")
+@pytest.mark.skipif(NO_SOURCES, reason="racon's sources not present (oracle/Makefile REF)")
 @pytest.mark.parametrize("shim_first", [False, True])
 def test_racons_cudabatch_builds_against_the_shim_with_the_documented_diff(tmp_path, shim_first):
     for f in ("cudabatch.hpp", "cudabatch.cpp"):
@@ -42,7 +45,7 @@ def test_racons_cudabatch_builds_against_the_shim_with_the_documented_diff(tmp_p
     assert res.returncode == 0, res.stderr[-3000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src", "cuda")), reason="reference sources not present")
+@pytest.mark.skipif(NO_SOURCES, reason="racon's sources not present (oracle/Makefile REF)")
 def test_racons_cudaaligner_builds_against_the_shim_with_the_documented_diff(tmp_path):
     """INTEGRATION.md section 5: racon's CUDABatchAligner (src/cuda/cudaaligner.{hpp,cpp}) over b200aln_aligner.hpp."""
     for f in ("cudaaligner.hpp", "cudaaligner.cpp"):

@@ -3,14 +3,14 @@
 Parity bar: bit-exact -- same edit distance, same operations (hence the same CIGAR) as edlib returns for
 edlibAlign(q, t, {-1, EDLIB_MODE_NW, EDLIB_TASK_PATH}) (src/overlap.cpp:205-224): the oracle's restatement on seeded
 random pairs around every threshold of edlib's recursion, the committed digests of the UNMODIFIED edlib on the 181
-real lambda-phage overlaps of the reference's test data, and oracle/_ref live where it travelled to the box."""
+real lambda-phage overlaps of the reference's test data, and its stored answers on long reads."""
 import hashlib
 
 import numpy as np
 import pytest
 
 from common import overlap_fixture, random_pairs
-from oracle_lib import ops_to_cigar, oracle_align, ref_align
+from oracle_lib import ops_to_cigar, oracle_align
 
 pytestmark = pytest.mark.gpu
 
@@ -241,9 +241,7 @@ def test_full_batch_is_back_pressure_not_an_error(oracle):
     assert info["cells"] > 0 and info["kernel_ms"] > 0
 
 
-def test_live_against_the_unmodified_edlib(ref, aligner):
-    if not ref.available:
-        pytest.skip("oracle/_ref not built (no /root/reference where it was built)")
+def unmodified_edlib_pairs():
     pairs = random_pairs(901, [(6000, 0.14), (2500, 0.3), (1900, 0.05), (64, 0.3)])
     # long reads: slots re-made for the longer sequences, five and more Hirschberg levels, huge sub-problems on teams at
     # several levels, leaves of many stripes (tall, narrow) -- only the real edlib is fast enough to check these
@@ -251,13 +249,18 @@ def test_live_against_the_unmodified_edlib(ref, aligner):
     rng = np.random.default_rng(5)
     pairs.append((rng.choice(ACGT, size=30000).tobytes(), rng.choice(ACGT, size=12000).tobytes()))  # unrelated, tall
     pairs.append((rng.choice(ACGT, size=900).tobytes(), rng.choice(ACGT, size=50000).tobytes()))    # unrelated, wide
+    return pairs
+
+
+def test_live_against_the_unmodified_edlib(ref, aligner):
+    pairs = unmodified_edlib_pairs()
     aligner.reset()
     for q, t in pairs:
         assert aligner.add_overlap(q, t)
     aligner.align_all()
     got = aligner.generate_cigar_strings()
     for k, (q, t) in enumerate(pairs):
-        ops, score, cigar = ref_align(ref, q, t)
+        ops, score, cigar = ref.align(q, t)
         assert got[k] == (cigar, score)
         assert (aligner.ops(k) == ops).all()
     aligner.reset()

@@ -2,8 +2,9 @@
 
 Parity target = spoa::Graph::generate_multiple_sequence_alignment (vendor/spoa/src/graph.cpp:373-427), which is what the
 reference's own test holds cudapoa's MSA against (vendor/GenomeWorks/cudapoa/tests/Test_CudapoaGenerateMSA2.cu:117-128).
-CPU here: the oracle's restatement against committed digests of the unmodified reference (tests/golden/ref_msa.npz),
-live against oracle/_ref, and the engine's emulation against the oracle.  GPU: tests/test_gpu_msa.py."""
+CPU here: the oracle's restatement against committed digests of the unmodified reference (tests/golden/ref_msa.npz)
+and its stored rows (tests/golden/ref_answers.npz), and the engine's emulation against the oracle.  GPU:
+tests/test_gpu_msa.py."""
 import os
 import sys
 
@@ -11,7 +12,7 @@ import numpy as np
 import pytest
 
 from common import G, GOLDEN, M, X
-from oracle_lib import oracle_window_msa, ref_window_msa
+from oracle_lib import oracle_window_msa
 
 sys.path.insert(0, GOLDEN)
 from make_msa_golden import digest, msa_groups  # noqa: E402
@@ -35,10 +36,8 @@ def test_oracle_msa_matches_the_committed_reference_digests(oracle, groups):
 
 
 def test_oracle_msa_matches_live_reference(oracle, ref, groups):
-    if not ref.available:
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
     for name, (seqs, wts, (m, x, g)) in list(groups.items())[:12]:
-        assert oracle_window_msa(oracle, seqs, wts, None, None, m, x, g) == ref_window_msa(ref, seqs, wts, m, x, g), name
+        assert oracle_window_msa(oracle, seqs, wts, None, None, m, x, g) == ref.window_msa(seqs, wts, m, x, g), name
 
 
 def _oracle_msas(oracle, b, order, m, x, g, spans=True):

@@ -31,9 +31,7 @@ def test_oracle_matches_reference_fixtures(oracle, name):
 
 
 def test_oracle_matches_live_reference(oracle, ref):
-    """Fresh seeds against oracle/_ref (only where /root/reference was available to build it)."""
-    if not ref.available:
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
+    """Fresh seeds against the unmodified reference (its stored answers)."""
     for (n, L, D, e, q, seed) in [(24, 500, 32, 0.15, False, 1), (24, 300, 12, 0.2, True, 2), (6, 1000, 40, 0.1, False, 3)]:
         b = synth_windows(n, L, D, e, seed=seed, with_quality=q)
         order = processing_order(b, ref.layer_order)
@@ -54,8 +52,6 @@ def test_oracle_matches_live_reference(oracle, ref):
 
 def test_partial_span_layers_use_the_subgraph_path(oracle, ref):
     """window.cpp:92-103: layers that do not span the window are aligned to a subgraph."""
-    if not ref.available:
-        pytest.skip("oracle/_ref not built")
     from common import partial_span_windows
     pb = partial_span_windows()
     order = processing_order(pb, ref.layer_order)
